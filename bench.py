@@ -4,7 +4,7 @@
 names — hash inner_join (configs[2]), groupby (configs[3]), scan / reduce — as sub-objects under `ops`, and (N > 1) the
 sharded inner_join (configs[4]) under `sharded_inner_join`.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--rows R] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--rows R] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one sort_by_key(values=T, keys=T) over a resident synthetic column (splitmix64 keys, SURVEY §8d); at N > 1
 the sharded sort (sample -> splitters -> range partition -> bucket exchange over NVLink -> local sort).
@@ -15,6 +15,9 @@ back to pinned host memory, every step, inside the timed region; the steps are s
 `cpu_baseline` / `--impl reference` time pandas (configs[0], the reference's CPU-runnable case) on a bounded 1e7-row
 sample of the same key stream on the host cores.
 Inputs (8 GB per GPU) are far larger than the 126 MB L2, so no explicit L2 flush is needed.
+`--dump-outputs DIR` writes the sorted column of the last timed step as DIR/sorted_keys.npy (float64; at N > 1 one file per
+rank, sorted_keys_rank<r>.npy): every row when the output fits DUMP_BYTES, else the rows at a fixed, seeded set of positions
+(ascending; see dump_sorted). The inputs depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -29,16 +32,26 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (which may be read-only)
 
 METRIC = "sort_by_key_rows_per_s"
 UNIT = "rows/s"
 SEED_KEYS = 0x5EED0001  # SURVEY §8d seed of the key stream (same constant as oracle/datagen.py; the GPU arm does not import oracle)
+DUMP_BYTES = 32 << 20  # --dump-outputs: float64 values per run, summed over ranks
+DUMP_SEED = 0x5EED00D0
+
+
+def _positive(s: str) -> int:
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=_positive, default=5, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--rows", type=int, default=1_000_000_000, help="rows per GPU")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -46,7 +59,11 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-ops", action="store_true", help="skip the per-operation measurements (join / groupby / scan / reduce) at N = 1")
     ap.add_argument("--no-join", action="store_true", help="skip the sharded inner_join measurement at N > 1")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the sorted column of the last timed step under DIR (.npy)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm times a CPU sample")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -196,6 +213,23 @@ def measured_traffic(kernel_key: str):
         return None, "no ncu capture of this kernel under profiles/ yet"
 
 
+def dump_sorted(out_dir: str, col, rank: int, world: int) -> None:
+    """Writes `col` (the int64 CUDA tensor a caller of the timed step receives) as float64 .npy under out_dir: all of it up to
+    cap = DUMP_BYTES // world // 8 rows, else its values at the ascending positions
+    np.unique(default_rng(DUMP_SEED + rank).integers(0, len(col), cap)), which depend only on the row count."""
+    import numpy as np
+    import torch
+
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    n, cap = col.numel(), DUMP_BYTES // world // 8
+    if n > cap:
+        rows = np.unique(np.random.default_rng(DUMP_SEED + rank).integers(0, n, cap))
+        col = col[torch.from_numpy(rows).to(col.device)]
+    name = "sorted_keys.npy" if world == 1 else f"sorted_keys_rank{rank}.npy"
+    np.save(d / name, col.cpu().numpy().astype(np.float64))
+
+
 def pin_to_gpu_numa_node(gpu_index: int):
     """Bind this process to the CPUs of the NUMA node its GPU hangs off, before the pinned host buffers are allocated (they are then
     placed on that node): the e2e copies of 8 ranks otherwise cross the host's socket interconnect. Returns a short note."""
@@ -291,11 +325,14 @@ def run_ours(args):
         barrier()
         e0.record(stream)
         for _ in range(args.steps):
+            out = None  # the previous step's output is released before this step allocates its own
             out = step()
-            del out
         e1.record(stream)
         barrier()
     _lib.lib.b2_profile_enable(0)
+    if args.dump_outputs:
+        dump_sorted(args.dump_outputs, out if world > 1 else out.columns()[0].to_torch(), rank, world)
+    del out
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     launches = _lib.kernel_launch_count() - launches0
     ms_step = ms_total / args.steps

@@ -12,6 +12,7 @@ HERE = Path(__file__).resolve().parent
 CSRC = HERE / "csrc"
 OBJ = HERE / "build"
 LIB = HERE / "libcudf_b200.so"
+STAMP = HERE / "libcudf_b200.stamp"
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
@@ -28,7 +29,19 @@ def _digest(paths) -> str:
     return h.hexdigest()
 
 
+def _inputs():
+    return sorted(CSRC.glob("*.cu")), sorted(CSRC.glob("*.cuh")) + [HERE.parent / "include" / "cudf_b200.h"]
+
+
+def _up_to_date() -> bool:
+    sources, headers = _inputs()
+    return LIB.exists() and STAMP.exists() and STAMP.read_text() == _digest(sources + headers)
+
+
 def build(force: bool = False, verbose: bool = False) -> Path:
+    # an up-to-date library is used as it is, without writing to the tree (which may be read-only)
+    if not force and _up_to_date():
+        return LIB
     # several ranks of a torchrun job may call build() at once: serialise them on a lock file
     import fcntl
 
@@ -42,13 +55,10 @@ def build(force: bool = False, verbose: bool = False) -> Path:
 
 
 def _build_locked(force: bool, verbose: bool) -> Path:
-    sources = sorted(CSRC.glob("*.cu"))
-    headers = sorted(CSRC.glob("*.cuh")) + [HERE.parent / "include" / "cudf_b200.h"]
-    OBJ.mkdir(exist_ok=True)
-    stamp = HERE / "libcudf_b200.stamp"
-    digest = _digest(sources + headers)
-    if not force and LIB.exists() and stamp.exists() and stamp.read_text() == digest:
+    if not force and _up_to_date():  # another rank built it while this one waited for the lock
         return LIB
+    sources, headers = _inputs()
+    digest = _digest(sources + headers)
     hdr_digest = _digest(headers)
 
     def compile_one(src: Path):
@@ -74,7 +84,7 @@ def _build_locked(force: bool, verbose: bool) -> Path:
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError(f"link failed:\n{r.stdout}\n{r.stderr}")
-    stamp.write_text(digest)
+    STAMP.write_text(digest)
     return LIB
 
 

@@ -79,8 +79,11 @@ def test_join_gold_maps():
 
 def test_murmur3_row_hash_pinned():
     """oracle/partition.py: MurmurHash3_x86_32 against the published known answers (SMHasher verification values) and against
-    scikit-learn's C implementation on random fixed-width values; hash_combine and the null hash against hand-computed values
-    (cpp/include/cudf/hashing/detail/hashing.hpp:83-86, row_operator/hashing.cuh:52-56)."""
+    scikit-learn's C implementation on random fixed-width values (tests/golden/murmur3_sklearn.npz: 300 values per dtype and
+    murmurhash3_32(value bytes, seed, positive=True) for seeds 0 and 619, computed with scikit-learn 1.9.0); hash_combine and the
+    null hash against hand-computed values (cpp/include/cudf/hashing/detail/hashing.hpp:83-86, row_operator/hashing.cuh:52-56)."""
+    from pathlib import Path
+
     import numpy as np
 
     from oracle import partition as op
@@ -89,17 +92,12 @@ def test_murmur3_row_hash_pinned():
              (np.uint16, 0x4321, 0, 0xA0F7B07A), (np.uint8, 0x21, 0, 0x72661CF4), (np.uint32, 0, 0, 0x2362F9DE)]
     for dt, v, seed, exp in known:
         assert int(op.murmur3_32_fixed(np.array([v], dt), seed)[0]) == exp
-    try:
-        from sklearn.utils import murmurhash3_32
-    except Exception:
-        murmurhash3_32 = None
-    if murmurhash3_32 is not None:
-        rng = np.random.default_rng(1)
-        for dt in (np.uint8, np.uint16, np.uint32, np.uint64, np.float32, np.float64):
-            v = rng.integers(0, 2**63 - 1, 300, dtype=np.int64).astype(dt) if np.dtype(dt).kind != "f" else rng.standard_normal(300).astype(dt)
-            for seed in (0, 619):
-                exp = np.array([murmurhash3_32(x.tobytes(), seed, positive=True) for x in v], dtype=np.uint32)
-                assert np.array_equal(op.murmur3_32_fixed(v, seed), exp)
+    gold = np.load(Path(__file__).resolve().parent / "golden" / "murmur3_sklearn.npz")
+    for dt in (np.uint8, np.uint16, np.uint32, np.uint64, np.float32, np.float64):
+        v = gold[f"{np.dtype(dt).name}_values"]
+        assert v.dtype == dt and len(v) == 300
+        for seed in (0, 619):
+            assert np.array_equal(op.murmur3_32_fixed(v, seed), gold[f"{np.dtype(dt).name}_seed{seed}"])
     # normalisation and nulls: -0.0 hashes like +0.0, every NaN like the canonical one, a null is UINT32_MAX
     f = np.array([0.0, -0.0, np.nan, -np.nan], np.float64)
     h = op.row_hash([(f, np.array([True, True, True, True]))])
